@@ -1,11 +1,15 @@
 #!/usr/bin/env python3
 """bench.py — PageRank GTEPS (edges/sec/iter) on synthetic RMAT, the headline metric of BASELINE.json.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--scale S] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one graph: `page_rank` with 20 forced sweeps
 (tolerance 0, damping 0.85) on the RMAT scale-S graph (default 26 = the configuration the metric is
 quoted on; it fits one B200).  One JSON line is printed by rank 0.
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float32, or float64 for
+integer results), so that two builds can be compared output for output: the inputs are generated from a
+fixed seed.  An output of more than 2**22 entries is cut to a fixed, seeded sample of its entries.
 
   value        m * sweeps * K / device time of K steps, graph resident in HBM, result left in HBM
   e2e          same metric through the C ABI with HOST buffers (gb_page_rank_csr_u32): every step uploads
@@ -122,6 +126,34 @@ def pinned_empty(count: int, dtype):
     return t, t.numpy().view(dtype)[:count]
 
 
+DUMP_SAMPLE = 1 << 22       # entries --dump-outputs keeps of one output array
+DUMP_BUDGET = 64 << 20      # bytes --dump-outputs may write in all
+
+
+def dump_index(n: int) -> np.ndarray:
+    """Sorted indices of the entries --dump-outputs keeps of an n-entry output: all of them up to
+    DUMP_SAMPLE, else a sample drawn from a fixed seed (the same indices on every run)."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.unique(np.random.default_rng(SEED).integers(0, n, DUMP_SAMPLE))
+
+
+def dump_outputs(path, outputs: dict) -> None:
+    """Writes every output as path/<name>.npy: float32 stays float32, everything else becomes float64
+    (exact for integers below 2**53)."""
+    arrays = {}
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        arrays[name] = a if a.dtype == np.float32 else a.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BUDGET} byte budget")
+    out = Path(path)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def algorithmic_bytes(n: int, m: int) -> int:
     return 4 * m + 24 * n + 4  # BASELINE.md §3 / SURVEY.md §8(d)
 
@@ -215,8 +247,10 @@ def run_reference(args):
         oracle.page_rank_mt(in_off, in_tgt, out_off, 1, 0.0, DAMPING, 0)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.page_rank_mt(in_off, in_tgt, out_off, sample_sweeps, 0.0, DAMPING, 0)
+        scores, it, err = oracle.page_rank_mt(in_off, in_tgt, out_off, sample_sweeps, 0.0, DAMPING, 0)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scores": scores[dump_index(n)], "iterations": [it], "error": [err]})
     gteps = m * sample_sweeps * args.steps / dt / 1e9
     sample = f"{sample_sweeps} of {SWEEPS} sweeps per step on the full RMAT scale-{scale} graph; input prep: {prep}"
     line = {
@@ -276,6 +310,9 @@ def run_single(args):
     ms = ev0.elapsed_time(ev1)
     assert it.value == SWEEPS
     gteps = m * SWEEPS * args.steps / (ms * 1e-3) / 1e9
+    if args.dump_outputs:   # taken before the passes below run the step again
+        idx = torch.from_numpy(dump_index(n)).to(d_scores.device)
+        outputs = {"scores": d_scores[idx].cpu().numpy(), "iterations": [it.value], "error": [err.value]}
 
     # dominant kernel, timed live with CUDA events around every launch (separate pass)
     lib.gb_set_profiling(1)
@@ -352,6 +389,8 @@ def run_single(args):
         "hbm_roofline_gteps": peak * 1e9 / (bytes_per_launch / m) / 1e9,
         "frac_of_hbm_roofline_whole_step": (bytes_per_launch * SWEEPS * args.steps / (ms * 1e-3) / 1e9) / peak,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
 
 
@@ -395,6 +434,9 @@ def run_multi(args):
     # untimed verification: the sharded ranks against a single-GPU run of the same graph on rank 0
     sharded = spr.scores_host()
     verified, verification = None, None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scores": sharded[dump_index(n)], "iterations": [spr.ran_iterations],
+                                         "error": [spr.error]})
     if rank == 0:
         single = g.page_rank(max_iterations=SWEEPS, tolerance=0.0, damping_factor=DAMPING, mode="jacobi").scores()
         worst = float(np.max(np.abs(sharded - single) / single))
@@ -477,7 +519,7 @@ def run_algo(args):
     torch.cuda.set_device(0)
     gb.set_device(0)
     peak, peak_src = peaks()
-    reps = max(args.steps, 3)
+    reps = args.steps
 
     def timed(fn):
         for _ in range(max(args.warmup, 1)):
@@ -501,6 +543,7 @@ def run_algo(args):
             res, dev_ms, wall_ms, launches = timed(lambda: g.wcc())
         byts = 8 * m + 16 * n + 8
         comp = res.components()
+        outputs = {"components": comp[dump_index(n)]}
         oo, ot = g.csr("out")
         io, it = g.csr("in")
         cpu = None
@@ -534,6 +577,7 @@ def run_algo(args):
             relabel_ms = (time.perf_counter() - t0) * 1e3
             res, dev_ms, wall_ms, launches = timed(lambda: g.global_triangle_count())
         launches += l0
+        outputs = {"triangles": [res.triangles]}
         byts = 8 * m + 4 * (n + 1)
         cpu, verified = None, None
         if not args.no_cpu:
@@ -565,6 +609,7 @@ def run_algo(args):
         with ClockSampler(0) as clocks:
             res, dev_ms, wall_ms, launches = timed(lambda: g.delta_stepping(start_node=start, delta=delta))
         d = res.distances()
+        outputs = {"distances": d[dump_index(n)]}
         byts = 8 * m + 4 * (n + 1) + 8 * n
         cpu, verified = None, None
         if not args.no_cpu:
@@ -591,6 +636,8 @@ def run_algo(args):
                  "scaling": "strong", "vs_baseline": None, "dtype": "u32" if args.algo != "sssp" else "f32",
                  "data": "synthetic", "clocks": clocks.summary(), "gpu_launches": int(launches),
                  "verified": verified, "cpu_baseline": cpu})
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
 
 
@@ -609,7 +656,11 @@ def main():
     ap.add_argument("--exchange", default="auto", choices=["auto", "peer", "allgather"])
     ap.add_argument("--no-multicast", action="store_true", help="multi-GPU: unicast peer stores instead of multimem.st")
     ap.add_argument("--diag", action="store_true", help="multi-GPU: print per-rank kernel / exchange ms per sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (larger outputs: a seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     elif args.algo != "page_rank":

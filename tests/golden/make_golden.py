@@ -1,18 +1,19 @@
 #!/usr/bin/env python3
-"""Regenerates tests/golden/ from the reference checkout (run in the build container only).
+"""Regenerates tests/golden/ from a checkout of neo4j-labs/graph:
+
+  python tests/golden/make_golden.py <path of the reference checkout>
 
 The Rust reference cannot be executed here (no cargo/rustc), so the golden OUTPUTS below are
 transcribed from the assertions of the reference's own tests — each entry carries the file:line
 it was read from — and the golden INPUT files are the reference's test resources, copied as data
-(they are binary/text fixtures, not source code).  `python tests/golden/make_golden.py` rewrites
-`reference_goldens.json` and refreshes the resource copies; nothing under tests/ reads
-/root/reference at test time.
+(they are binary/text fixtures, not source code).  It rewrites `reference_goldens.json` and refreshes
+the resource copies; nothing under tests/ reads the reference checkout at test time.
 """
 import json
 import shutil
+import sys
 from pathlib import Path
 
-REF = Path("/root/reference")
 HERE = Path(__file__).resolve().parent
 
 RESOURCES = ["scale_8.graph500", "test.el", "example.el", "test.wel", "example.wel", "windows.el"]
@@ -138,8 +139,11 @@ GOLDENS = {
 
 
 def main():
+    if len(sys.argv) != 2:
+        sys.exit(f"usage: {sys.argv[0]} <path of the reference checkout>")
+    ref = Path(sys.argv[1])
     for name in RESOURCES:
-        shutil.copyfile(REF / "resources" / name, HERE / name)
+        shutil.copyfile(ref / "resources" / name, HERE / name)
     (HERE / "reference_goldens.json").write_text(json.dumps(GOLDENS, indent=1) + "\n")
     print("wrote", HERE / "reference_goldens.json")
 

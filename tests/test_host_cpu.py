@@ -56,7 +56,7 @@ def test_product_never_imports_the_oracle():
         assert "import oracle" not in src and "from oracle" not in src, path
 
 
-def test_graph500_reader_matches_reference_format(golden_dir, goldens):
+def test_graph500_reader_matches_reference_format(golden_dir, goldens, tmp_path):
     import graph_b200 as gb
     import oracle
     src, dst, n = gb._read_graph500(golden_dir / "scale_8.graph500")
@@ -64,13 +64,10 @@ def test_graph500_reader_matches_reference_format(golden_dir, goldens):
     assert n == on == 256 and (src == osrc).all() and (dst == odst).all()
     # ids above 32 bits are rejected like Idx::new (index.rs:51-54)
     bad = np.array([1, 2, 0x00010000], dtype="<u4")
-    p = golden_dir.parent / "_tmp_bad.graph500"
+    p = tmp_path / "bad.graph500"
     bad.tofile(p)
-    try:
-        with pytest.raises(ValueError):
-            gb._read_graph500(p)
-    finally:
-        p.unlink()
+    with pytest.raises(ValueError):
+        gb._read_graph500(p)
 
 
 def test_edge_list_reader(golden_dir):
