@@ -125,10 +125,6 @@ struct PrPlan {
   uint32_t fin_hub_ctas = 0; // finish CTAs that take the hub groups (the others take rows [n_fin_warp, n_fin))
   uint32_t n_fin = 0;        // rows [0, n_fin) are completed by k_pr_finish, [n_fin, n_cb) by k_pr_sell
   uint32_t few_nrows[SELL_FEW] = {}, few_poff[SELL_FEW] = {};
-  // dual mode: k_pr_cb and k_pr_sell run at the same time on the same SMs (two streams, 512-thread CTAs)
-  bool dual = false;
-  cudaStream_t s2 = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   DevBuf<double> block_err;  // per CTA error partials (SELL CTAs, then finish CTAs)
   DevBuf<double> err_hist;   // error of each sweep of the current batch
   DevBuf<uint32_t> ctrl;     // [0] = done flag (sweep number at which tolerance was met), [1] = ticket
@@ -163,9 +159,6 @@ void free_pr_plan(PrPlan* p) {
   }
   for (cudaEvent_t e : p->trace_events) cudaEventDestroy(e);
   for (cudaEvent_t e : p->prof_events) cudaEventDestroy(e);
-  if (p->ev_fork) cudaEventDestroy(p->ev_fork);
-  if (p->ev_join) cudaEventDestroy(p->ev_join);
-  if (p->s2) cudaStreamDestroy(p->s2);
   delete p;
 }
 uint64_t pr_plan_bytes(const PrPlan* p) { return p ? p->bytes() : 0; }
@@ -249,11 +242,9 @@ __global__ void k_blk_edges(const uint32_t* __restrict__ outdeg, uint32_t n, uin
     blk_edges[b] = t;
   }
 }
-// rows_ge[b] = number of (global) rows with in-degree >= dmin[b] (indeg is non-increasing);
-// edges_ge[b] = the in-edges of those rows (deg_prefix = inclusive prefix sums of indeg)
-__global__ void k_rows_ge(const uint32_t* __restrict__ indeg, const unsigned long long* __restrict__ deg_prefix,
-                          uint32_t n_active, const uint32_t* __restrict__ dmin, uint32_t nblk,
-                          uint32_t* __restrict__ rows_ge, unsigned long long* __restrict__ edges_ge) {
+// rows_ge[b] = number of (global) rows with in-degree >= dmin[b] (indeg is non-increasing)
+__global__ void k_rows_ge(const uint32_t* __restrict__ indeg, uint32_t n_active, const uint32_t* __restrict__ dmin,
+                          uint32_t nblk, uint32_t* __restrict__ rows_ge) {
   for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < nblk; b += gridDim.x * blockDim.x) {
     const uint32_t d = dmin[b];
     uint32_t lo = 0, hi = n_active;  // first index with indeg < d
@@ -263,12 +254,8 @@ __global__ void k_rows_ge(const uint32_t* __restrict__ indeg, const unsigned lon
       else hi = mid;
     }
     rows_ge[b] = lo;
-    edges_ge[b] = lo ? deg_prefix[lo - 1] : 0ull;
   }
 }
-struct U32ToU64 {
-  __host__ __device__ unsigned long long operator()(uint32_t v) const { return v; }
-};
 
 // Classification of the in-edges of the rows that own segments (local rows [n_mega, n_cb)).  An edge
 // from source s (internal id) lands in block s / B; if that block is hot (rank j) and the row is inside
@@ -669,8 +656,7 @@ struct PrArgs {
   uint32_t n_fin;       // rows [0, n_fin) are completed by k_pr_finish (rem[] + partials); rows [n_fin, n_cb) own
                         // segments in at most SELL_FEW blocks and are completed by their k_pr_sell lane
   uint32_t few_kb, few_nrows[SELL_FEW], few_poff[SELL_FEW];  // the first blocks' row prefixes / partial offsets
-  uint32_t dbg;         // GB_PR_DEBUG bits (diagnostics): 1 = SELL slices CTA-major, 2 = static chunk->warp map, 4 = no TMA
-  uint32_t fix_in_sell; // k_pr_sell adds the parts of cut segments first (sequential mode: no k_pr_fixup launch)
+  uint32_t fix_in_sell; // k_pr_sell adds the parts of cut segments first (no k_pr_fixup launch)
   const uint32_t* fin_kb;  // [ceil(n_cb / 32)] blocks in which the first row of each 32-row group owns a segment
   // column blocks
   uint32_t B, KB;
@@ -878,8 +864,7 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst_smem, const void* src, uin
 // thin blocks are (a purely static split ran 2.4x slower, one global cursor reloads the block for every
 // task: profiles/r02_sweep_breakdown.txt).  Claiming the next task one task ahead (to hide the atomic's
 // round trip) was measured and dropped: a claimed task cannot be stolen, which costs more at the tail.
-template <int NT>
-__device__ __forceinline__ void pr_cb_body(const PrArgs& a) {
+__global__ void __launch_bounds__(PR_THREADS, 1) k_pr_cb(const PrArgs a) {
   extern __shared__ __align__(128) float smem[];
   float* xs = smem;  // B entries of x_cur + one zero slot (the pad id)
   __shared__ uint32_t s_task, s_next;
@@ -891,7 +876,7 @@ __device__ __forceinline__ void pr_cb_body(const PrArgs& a) {
   const uint32_t R = gridDim.x;  // ranges = CTAs
   const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&s_mbar);
   const uint32_t xs_smem = (uint32_t)__cvta_generic_to_shared(xs);
-  const bool bulk_ok = (reinterpret_cast<uintptr_t>(a.x_cur) & 15u) == 0 && !(a.dbg & 4u);  // cp.async.bulk moves 16-byte units
+  const bool bulk_ok = (reinterpret_cast<uintptr_t>(a.x_cur) & 15u) == 0;  // cp.async.bulk moves 16-byte units
   uint32_t phase = 0;
   if (threadIdx.x == 0) mbar_init(mbar, 1);
   if (threadIdx.x < 4) xs[B + threadIdx.x] = 0.0f;  // the pad id's zero slot: never overwritten
@@ -930,7 +915,7 @@ __device__ __forceinline__ void pr_cb_body(const PrArgs& a) {
     }
     __syncthreads();  // also: every warp is done with the previous task's block
     const uint32_t t = s_task;
-    if (threadIdx.x == 0) s_next = NT / 32;  // every warp is past its last claim of the previous task
+    if (threadIdx.x == 0) s_next = PR_WARPS;  // every warp is past its last claim of the previous task
     __syncthreads();
     if (t == CB_NONE) break;
     const uint2 task = a.tasks[t];  // (first chunk, chunk count | block rank << 8)
@@ -950,7 +935,7 @@ __device__ __forceinline__ void pr_cb_body(const PrArgs& a) {
         mbar_wait(mbar, phase);
         phase ^= 1u;
       } else {
-        for (uint32_t i = threadIdx.x; i < cnt; i += NT) xs[i] = a.x_cur[x0 + i];
+        for (uint32_t i = threadIdx.x; i < cnt; i += PR_THREADS) xs[i] = a.x_cur[x0 + i];
       }
       cur_j = j;
       __syncthreads();
@@ -961,14 +946,10 @@ __device__ __forceinline__ void pr_cb_body(const PrArgs& a) {
       cb_chunk(a, xs, task.x + k, lane, pad2);
       uint32_t nx = 0;
       if (lane == 0) nx = atomicAdd(&s_next, 1u);
-      k = (a.dbg & 2u) ? k + NT / 32 : __shfl_sync(0xFFFFFFFFu, nx, 0);
+      k = __shfl_sync(0xFFFFFFFFu, nx, 0);
     }
   }
 }
-__global__ void __launch_bounds__(PR_THREADS, 1) k_pr_cb(const PrArgs a) { pr_cb_body<PR_THREADS>(a); }
-// dual mode: 512 threads and at most 56 registers, so that a 512-thread k_pr_sell CTA (64 registers)
-// fits beside it on the SM
-__global__ void __maxnreg__(56) k_pr_cb_half(const PrArgs a) { pr_cb_body<PR_THREADS / 2>(a); }
 
 // Segments cut by chunk boundaries (segments longer than a chunk): one warp per segment adds its parts
 // in a fixed order — the head part of the first chunk, then lanes over the following chunks (a fixed
@@ -999,8 +980,7 @@ __global__ void k_pr_fixup(const PrArgs a) {
 // lane-minor), gathers, and adds in row order.  The next slice's first targets and row metadata are
 // requested while the current slice is processed.  Rows below n_cb only hold the edges that are not in
 // a column-block segment: their sum goes to rem[] and the finish kernel completes them.
-// The kernel needs no shared memory: two 512-thread CTAs per SM when it runs alone, one beside a
-// k_pr_cb_half CTA in dual mode.
+// The kernel needs no shared memory: two 512-thread CTAs per SM.
 template <bool PEERS>
 __global__ void __launch_bounds__(PR_SELL_THREADS, 2) k_pr_sell(const PrArgs a) {
   constexpr int NT = PR_SELL_THREADS;
@@ -1020,7 +1000,7 @@ __global__ void __launch_bounds__(PR_SELL_THREADS, 2) k_pr_sell(const PrArgs a) 
   const uint32_t P = a.deal.P, pp = a.deal.p;
   // slices are dealt CTA-minor: the widest slices (the first ones) land on different SMs, not on the 16
   // warps of CTA 0 (an eighth-shard ran with its busiest SM 31 % above the average otherwise)
-  uint32_t sidx = (a.dbg & 1u) ? blockIdx.x * NW + warp : warp * gridDim.x + blockIdx.x;
+  uint32_t sidx = warp * gridDim.x + blockIdx.x;
   // pipeline state: metadata of this and the next slice, first two target groups + row data of this one
   uint2 meta = make_uint2(0, 0), nmeta = meta;
   uint4 ta = pad, tb = pad;
@@ -1442,22 +1422,11 @@ static gb_status build_pr_plan(const gb_graph* g, PrDeal deal, PrPlan** out_plan
     uint32_t n_mega = 0;  // local rows [0, n_mega) are long enough for the sort path of the build
     std::vector<uint32_t> h_hot(nblk, CB_NONE), h_blk, h_nrows, h_poff;
     if (p->n_loc && m) {
-      DevBuf<unsigned long long> blk_edges, deg_prefix, edges_ge;
+      DevBuf<unsigned long long> blk_edges;
       DevBuf<uint32_t> dmin, rows_ge;
       GB_TRY(blk_edges.alloc(nblk));
       GB_TRY(dmin.alloc(nblk + 1));  // + one probe: the rows long enough for the sort path of the build
       GB_TRY(rows_ge.alloc(nblk + 1));
-      GB_TRY(edges_ge.alloc(nblk + 1));
-      GB_TRY(deg_prefix.alloc(std::max<uint32_t>(p->n_active, 1)));
-      {
-        cub::TransformInputIterator<unsigned long long, U32ToU64, const uint32_t*> it(indeg.p, U32ToU64());
-        size_t tb = 0;
-        GB_CUDA(cub::DeviceScan::InclusiveSum(nullptr, tb, it, deg_prefix.p, (int)p->n_active, s));
-        DevBuf<uint8_t> tmp;
-        GB_TRY(tmp.alloc(tb));
-        GB_CUDA(cub::DeviceScan::InclusiveSum(tmp.p, tb, it, deg_prefix.p, (int)p->n_active, s));
-        GB_CUDA(cudaStreamSynchronize(s));
-      }
       k_blk_edges<<<nblk, 256, 0, s>>>(p->outdeg.p, n, B, blk_edges.p);
       std::vector<unsigned long long> h_edges(nblk);
       GB_CUDA(cudaMemcpyAsync(h_edges.data(), blk_edges.p, (size_t)nblk * 8, cudaMemcpyDeviceToHost, s));
@@ -1470,26 +1439,17 @@ static gb_status build_pr_plan(const gb_graph* g, PrDeal deal, PrPlan** out_plan
           h_dmin[b] = d >= 4294967295.0 ? 0xFFFFFFFFu : std::max<uint32_t>(1u, (uint32_t)d);
         }
       GB_CUDA(cudaMemcpyAsync(dmin.p, h_dmin.data(), (size_t)(nblk + 1) * 4, cudaMemcpyHostToDevice, s));
-      k_rows_ge<<<grid_for(nblk + 1, 128), 128, 0, s>>>(indeg.p, deg_prefix.p, p->n_active, dmin.p, nblk + 1, rows_ge.p,
-                                                         edges_ge.p);
+      k_rows_ge<<<grid_for(nblk + 1, 128), 128, 0, s>>>(indeg.p, p->n_active, dmin.p, nblk + 1, rows_ge.p);
       std::vector<uint32_t> h_rows(nblk + 1);
-      std::vector<unsigned long long> h_ege(nblk + 1);
       GB_CUDA(cudaMemcpyAsync(h_rows.data(), rows_ge.p, (size_t)(nblk + 1) * 4, cudaMemcpyDeviceToHost, s));
-      GB_CUDA(cudaMemcpyAsync(h_ege.data(), edges_ge.p, (size_t)(nblk + 1) * 8, cudaMemcpyDeviceToHost, s));
       GB_CUDA(cudaStreamSynchronize(s));
       n_mega = deal_count(h_rows[nblk], deal.P, deal.p);
-      // GB_PR_MIN_BLOCK (experiment): drop blocks whose segments are expected to hold fewer ids than this
-      // (this shard's share of: in-edges of the qualifying rows x the block's share of all gathers).
-      // Default 0: a thin block costs one block load (~2 us on one SM), while its ids would otherwise
-      // lengthen the SELL lanes of the hub rows, which one lane walks serially.
-      double min_ids = 0.0;
-      if (const char* e = getenv("GB_PR_MIN_BLOCK")) min_ids = atof(e);
+      // every block with a qualifying local row is kept, however thin: a thin block costs one block load
+      // (~2 us on one SM), while its ids would otherwise lengthen the SELL lanes of the hub rows, which
+      // one lane walks serially
       std::vector<uint32_t> order;
-      for (uint32_t b = 0; b < nblk; ++b) {
-        if (h_dmin[b] == 0xFFFFFFFFu || deal_count(h_rows[b], deal.P, deal.p) == 0) continue;
-        const double expect = (double)h_ege[b] * ((double)h_edges[b] / (double)m) / (double)deal.P;
-        if (expect >= min_ids) order.push_back(b);
-      }
+      for (uint32_t b = 0; b < nblk; ++b)
+        if (h_dmin[b] != 0xFFFFFFFFu && deal_count(h_rows[b], deal.P, deal.p) != 0) order.push_back(b);
       std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) {
         return h_rows[x] != h_rows[y] ? h_rows[x] > h_rows[y] : x < y;
       });
@@ -1690,7 +1650,7 @@ static gb_status build_pr_plan(const gb_graph* g, PrDeal deal, PrPlan** out_plan
       // >= 64 chunks (down to one 64-group step each) so that all warps share it — a lone warp runs at
       // its dependency latency, ~10x below the SM's throughput
       uint32_t C = env_u32("GB_PR_CHUNK", 0);
-      const uint32_t T = std::min<uint32_t>(std::max<uint32_t>(env_u32("GB_PR_TASK_CHUNKS", CB_TASK_CHUNKS), 32u), 128u);
+      const uint32_t T = CB_TASK_CHUNKS;
       if (!C) C = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(p->NG / ((uint64_t)dev_sms * 8 * T), 16384 / T), 65536 / T);
       C = std::max<uint32_t>(32u, (C + 31) / 32 * 32);
       p->chunk_groups = C;
@@ -1747,21 +1707,11 @@ static gb_status build_pr_plan(const gb_graph* g, PrDeal deal, PrPlan** out_plan
     // 8. launch shapes and error buffers
     p->smem_cb = ((size_t)B + 4) * sizeof(float);
     GB_CUDA(cudaFuncSetAttribute(k_pr_cb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_cb));
-    GB_CUDA(cudaFuncSetAttribute(k_pr_cb_half, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->smem_cb));
-    // GB_PR_DUAL=1 (experiment): k_pr_cb_half and k_pr_sell at the same time on two streams.  Measured
-    // (profiles/r02_sweep_breakdown.txt): both kernels load the same LSU data pipe, so the overlap buys
-    // <= 5 % at a 128 KB block and loses with larger blocks (k_pr_sell then starves for L1); default off.
-    p->dual = p->grid_cb > 0 && p->num_slices > 0 && env_u32("GB_PR_DUAL", 0) != 0;
-    if (p->dual) {
-      GB_CUDA(cudaStreamCreateWithFlags(&p->s2, cudaStreamNonBlocking));
-      GB_CUDA(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
-      GB_CUDA(cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming));
-    }
     const uint64_t want_sell = ((uint64_t)p->num_slices + PR_SELL_THREADS / 32 - 1) / (PR_SELL_THREADS / 32);
     p->grid_sell = (unsigned)std::min<uint64_t>(want_sell, (uint64_t)dev_sms * 2);
     // rows with segments in more than SELL_FEW blocks are a prefix (nrows[] is non-increasing): k_pr_finish
-    // completes them; all others are completed by their k_pr_sell lane (sequential mode: k_pr_cb is done by then)
-    p->n_fin = p->dual ? p->n_cb : (p->KB > SELL_FEW ? std::min<uint32_t>(p->n_cb, (h_nrows[SELL_FEW] + 31) / 32 * 32) : 0);
+    // completes them; all others are completed by their k_pr_sell lane (k_pr_cb is done by then)
+    p->n_fin = p->KB > SELL_FEW ? std::min<uint32_t>(p->n_cb, (h_nrows[SELL_FEW] + 31) / 32 * 32) : 0;
     for (uint32_t j = 0; j < SELL_FEW && j < p->KB; ++j) {
       p->few_nrows[j] = h_nrows[j];
       p->few_poff[j] = h_poff[j];
@@ -1804,7 +1754,7 @@ static gb_status build_pr_plan(const gb_graph* g, PrDeal deal, PrPlan** out_plan
 // row is completed later, by k_pr_finish (rows below n_fin).  A row that its k_pr_sell lane completes itself
 // (few hot blocks: small graphs) needs the sum BEFORE that kernel: k_pr_fixup runs in between.
 static bool fix_in_sell(const PrPlan* p) {
-  return !p->dual && p->n_fix && p->grid_sell && p->fix_max_row < p->n_fin;
+  return p->n_fix && p->grid_sell && p->fix_max_row < p->n_fin;
 }
 static PrArgs make_args(const PrPlan* p, float base, float damping, double tolerance) {
   PrArgs a{};
@@ -1822,7 +1772,6 @@ static PrArgs make_args(const PrPlan* p, float base, float damping, double toler
     a.few_poff[j] = p->few_poff[j];
   }
   a.fix_in_sell = fix_in_sell(p) ? 1u : 0u;
-  a.dbg = env_u32("GB_PR_DEBUG", 0);
   a.B = p->B;
   a.KB = p->KB;
   a.blk = p->blk.p;
@@ -1858,52 +1807,36 @@ static PrArgs make_args(const PrPlan* p, float base, float damping, double toler
   return a;
 }
 
-// one sweep = column blocks (+ fixup of cut segments) and SELL rows — at the same time in dual mode —
-// then finish; *launches is advanced by the kernels launched
+// one sweep = column blocks (+ fixup of cut segments), SELL rows, then finish; *launches is advanced by
+// the kernels launched
 template <bool PEERS>
 static gb_status launch_sweep(const PrPlan* p, const PrArgs& a, cudaStream_t s, uint64_t* launches) {
-  const unsigned fix_grid = grid_for((uint64_t)p->n_fix * 32, 128, 296);
-  if (p->dual) {
-    GB_CUDA(cudaEventRecord(p->ev_fork, s));
-    GB_CUDA(cudaStreamWaitEvent(p->s2, p->ev_fork, 0));
-    k_pr_cb_half<<<p->grid_cb, PR_THREADS / 2, p->smem_cb, s>>>(a);
-    k_pr_sell<PEERS><<<p->grid_sell, PR_SELL_THREADS, 0, p->s2>>>(a);
-    if (p->n_fix) k_pr_fixup<<<fix_grid, 128, 0, s>>>(a);
-    GB_CUDA(cudaEventRecord(p->ev_join, p->s2));
-    GB_CUDA(cudaStreamWaitEvent(s, p->ev_join, 0));
-    *launches += 2 + (p->n_fix ? 1 : 0);
-  } else {
-    cudaEvent_t* ev = nullptr;
-    if (p->trace && p->trace_events.size() < 5 * 256) {
-      const size_t base = p->trace_events.size();
-      p->trace_events.resize(base + 5);
-      for (int k = 0; k < 5; ++k) GB_CUDA(cudaEventCreate(&p->trace_events[base + k]));
-      ev = &p->trace_events[base];
-      GB_CUDA(cudaEventRecord(ev[0], s));
-    }
-    if (p->grid_cb) {
-      k_pr_cb<<<p->grid_cb, PR_THREADS, p->smem_cb, s>>>(a);
-      if (ev) GB_CUDA(cudaEventRecord(ev[1], s));
-      if (p->n_fix && !a.fix_in_sell) k_pr_fixup<<<fix_grid, 128, 0, s>>>(a);
-      *launches += 1 + (p->n_fix && !a.fix_in_sell ? 1 : 0);
-    } else if (ev) {
-      GB_CUDA(cudaEventRecord(ev[1], s));
-    }
-    if (ev) GB_CUDA(cudaEventRecord(ev[2], s));
-    if (p->grid_sell) {
-      k_pr_sell<PEERS><<<p->grid_sell, PR_SELL_THREADS, 0, s>>>(a);
-      *launches += 1;
-    }
-    if (ev) GB_CUDA(cudaEventRecord(ev[3], s));
-    if (p->fin_u == 2) k_pr_finish<PEERS, 2><<<p->grid_fin, PR_FIN_THREADS, 0, s>>>(a);
-    else k_pr_finish<PEERS, 4><<<p->grid_fin, PR_FIN_THREADS, 0, s>>>(a);
-    if (ev) GB_CUDA(cudaEventRecord(ev[4], s));
-    *launches += 1;
-    GB_CUDA(cudaGetLastError());
-    return GB_OK;
+  cudaEvent_t* ev = nullptr;
+  if (p->trace && p->trace_events.size() < 5 * 256) {
+    const size_t base = p->trace_events.size();
+    p->trace_events.resize(base + 5);
+    for (int k = 0; k < 5; ++k) GB_CUDA(cudaEventCreate(&p->trace_events[base + k]));
+    ev = &p->trace_events[base];
+    GB_CUDA(cudaEventRecord(ev[0], s));
   }
+  if (p->grid_cb) {
+    k_pr_cb<<<p->grid_cb, PR_THREADS, p->smem_cb, s>>>(a);
+    *launches += 1;
+  }
+  if (ev) GB_CUDA(cudaEventRecord(ev[1], s));
+  if (p->n_fix && !a.fix_in_sell) {  // n_fix > 0 implies column blocks, so k_pr_cb ran
+    k_pr_fixup<<<grid_for((uint64_t)p->n_fix * 32, 128, 296), 128, 0, s>>>(a);
+    *launches += 1;
+  }
+  if (ev) GB_CUDA(cudaEventRecord(ev[2], s));
+  if (p->grid_sell) {
+    k_pr_sell<PEERS><<<p->grid_sell, PR_SELL_THREADS, 0, s>>>(a);
+    *launches += 1;
+  }
+  if (ev) GB_CUDA(cudaEventRecord(ev[3], s));
   if (p->fin_u == 2) k_pr_finish<PEERS, 2><<<p->grid_fin, PR_FIN_THREADS, 0, s>>>(a);
   else k_pr_finish<PEERS, 4><<<p->grid_fin, PR_FIN_THREADS, 0, s>>>(a);
+  if (ev) GB_CUDA(cudaEventRecord(ev[4], s));
   *launches += 1;
   GB_CUDA(cudaGetLastError());
   return GB_OK;

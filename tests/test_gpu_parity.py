@@ -603,7 +603,6 @@ def test_page_rank_column_block_knobs(gb, monkeypatch, block, chunk, tau):
     monkeypatch.setenv("GB_PR_BLOCK", str(block))
     monkeypatch.setenv("GB_PR_CHUNK", str(chunk))
     monkeypatch.setenv("GB_PR_TAU", str(tau))
-    monkeypatch.setenv("GB_PR_MIN_BLOCK", "0")    # keep even the thinnest blocks
     monkeypatch.setenv("GB_PR_MEGA", "200")       # rows above 200 in-edges take the sort path of the layout build
     src, dst = oracle.rmat_edges(16, seed=5)
     n = 1 << 16

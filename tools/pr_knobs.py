@@ -32,7 +32,7 @@ def main():
     cfg = _capi.PageRankConfig(20, 0.0, 0.85, _capi.PR_JACOBI)
     it, err = C.c_uint64(0), C.c_double(0.0)
     peak = json.loads((ROOT / "MEASURED_PEAKS.json").read_text())["hbm_gbs"] if (ROOT / "MEASURED_PEAKS.json").exists() else 6650.0
-    names = {"B": "GB_PR_BLOCK", "TAU": "GB_PR_TAU", "CHUNK": "GB_PR_CHUNK", "MINB": "GB_PR_MIN_BLOCK", "DUAL": "GB_PR_DUAL", "TASK": "GB_PR_TASK_CHUNKS"}
+    names = {"B": "GB_PR_BLOCK", "TAU": "GB_PR_TAU", "CHUNK": "GB_PR_CHUNK"}
     for conf in args.configs.split(";"):
         for k in names.values():
             os.environ.pop(k, None)
